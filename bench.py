@@ -114,6 +114,53 @@ class ClockSampler(threading.Thread):
                 "samples": len(rows), "sm_min_mhz": min(sm) if sm else None, "timed_regions": len(self.windows)}
 
 
+DUMP_SAMPLE_BYTES = 4 << 20  # output bytes kept by --dump-outputs per run: 16 MiB of values + 32 MiB of positions
+
+
+def dump_outputs(jobs, out_dir, rank, world):
+    """--dump-outputs: what a caller of the timed path receives from its last step, as .npy files that two builds can be compared on.
+    file_meta (float64, one row per output file of every job): the job's index, then the numeric fields of FileMeta in header order;
+    output_keys (float32 [files, 2, 64]): the bytes of the smallest and the largest internal key (zero padded);
+    job_stats (float64, one row per job): the counters of JobStats (its timings are left out: they change from run to run);
+    output_bytes (float32) at output_byte_positions (float64): the bytes of the output tables laid end to end, all of them or a
+    seeded sample of DUMP_SAMPLE_BYTES positions, so that the whole dump stays under 64 MB."""
+    import numpy as np
+    import torch
+    from toplingdb_b200.native import FileMeta, JobStats
+    if world > 1:
+        out_dir = os.path.join(out_dir, f"rank{rank}")
+    os.makedirs(out_dir, exist_ok=True)
+    files = [(jx, j, i, j.output_meta(i)) for jx, j in enumerate(jobs) for i in range(j.output_count())]
+    meta_fields = [n for n, _ in FileMeta._fields_ if not n.endswith("_ikey")]
+    meta = [[jx] + [getattr(m, n) for n in meta_fields] for jx, _, _, m in files]
+    keys = np.zeros((len(files), 2, 64), dtype=np.float32)
+    for f, (_, _, _, m) in enumerate(files):
+        keys[f, 0] = list(m.smallest_ikey)
+        keys[f, 1] = list(m.largest_ikey)
+        keys[f, 0, min(m.smallest_ikey_len, 64):] = 0
+        keys[f, 1, min(m.largest_ikey_len, 64):] = 0
+    stat_fields = [n for n, _ in JobStats._fields_ if not n.endswith("_us")]
+    stats = [[getattr(s, n) for n in stat_fields] for s in (j.stats() for j in jobs)]
+    sizes = np.array([m.file_size for _, _, _, m in files], dtype=np.int64)
+    starts = np.concatenate([[0], np.cumsum(sizes)])
+    n_sample = DUMP_SAMPLE_BYTES // world
+    if starts[-1] <= n_sample:
+        pos = np.arange(starts[-1], dtype=np.int64)
+    else:
+        pos = np.sort(np.random.default_rng(0).integers(0, starts[-1], n_sample))
+    vals = []
+    for f, (_, j, i, m) in enumerate(files):
+        lo, hi = np.searchsorted(pos, [starts[f], starts[f + 1]])
+        img = torch.empty(m.file_size, dtype=torch.uint8, device=torch.device("cuda", j.params.device))
+        j.output_read_into(i, img)
+        vals.append(img[torch.from_numpy(pos[lo:hi] - starts[f]).to(img.device)].cpu().numpy())
+    np.save(os.path.join(out_dir, "file_meta.npy"), np.array(meta, dtype=np.float64).reshape(len(files), 1 + len(meta_fields)))
+    np.save(os.path.join(out_dir, "output_keys.npy"), keys)
+    np.save(os.path.join(out_dir, "job_stats.npy"), np.array(stats, dtype=np.float64))
+    np.save(os.path.join(out_dir, "output_bytes.npy"), np.concatenate(vals or [np.zeros(0, np.uint8)]).astype(np.float32))
+    np.save(os.path.join(out_dir, "output_byte_positions.npy"), pos.astype(np.float64))
+
+
 def reference_arm(args, rank, world):
     """The reference's own CPU ProcessKeyValueCompaction (oracle/_ref = the unmodified reference compiled here; else the
     CPU oracle port), all host threads, on a bounded sample of the same workload."""
@@ -235,6 +282,8 @@ def concurrent_jobs_arm(args, w, rank, world, local, numa_info):
     nout = sum(j.output_count() for j in jobs)
     launches = sum(j.stats().kernel_launches for j in jobs)
     kern = [{"name": n, "us": round(us, 1)} for n, us in jobs[0].kernel_times()]
+    if args.dump_outputs:
+        dump_outputs(jobs, args.dump_outputs, rank, world)
     if world > 1:
         tt = torch.tensor([step_s, wall_s], dtype=torch.float64, device="cuda")
         dist.all_reduce(tt, op=dist.ReduceOp.MAX)
@@ -306,7 +355,12 @@ def main():
     ap.add_argument("--e2e-depth", type=int, default=4, help="compaction jobs in flight in the end-to-end measurement")
     ap.add_argument("--no-numa", action="store_true", help="do not bind the rank to its GPU's NUMA node")
     ap.add_argument("--pipeline-ranges", type=int, default=8, help="key ranges of the pipelined single-job measurement (e2e.single_job_pipelined)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step to DIR/*.npy (see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the CUDA path (--impl b200)")
     rank = int(os.environ.get("RANK", 0))
     world = int(os.environ.get("WORLD_SIZE", 1))
     local = int(os.environ.get("LOCAL_RANK", 0))
@@ -408,6 +462,8 @@ def main():
         a, b = bytes(m.smallest_ikey[:16]), bytes(m.largest_ikey[:16])
         assert a <= b and (prev is None or prev < a), "output files out of order"
         prev = b
+    if args.dump_outputs:
+        dump_outputs([job], args.dump_outputs, rank, world)
 
     # per-kernel roofline on the dominant kernel group
     pk, pk_src = peaks()

@@ -56,13 +56,13 @@ def test_product_does_not_reference_the_oracle():
 
 
 @pytest.mark.skipif(not (os.path.exists(H.REF_BIN) and os.path.exists(H.REF_B200_BIN)), reason="oracle/_ref not built")
-def test_plugin_without_a_device_lets_the_reference_run_the_job_itself():
+def test_plugin_without_a_device_lets_the_reference_run_the_job_itself(monkeypatch):
     """No CUDA device: B200CompactionExecutorFactory::ShouldRunLocal() must answer true (compaction_executor.h:162), so the
     reference's CompactionJob::Run takes RunLocal() (compaction_job.cc:645-647) -- the plugin never computes anything on
-    the CPU itself.  Same files as a run without the plugin, and no remote-compaction bytes accounted."""
+    the CPU itself.  Same files as a run without the plugin, and no remote-compaction bytes accounted.  Any CUDA device is hidden
+    from the reference (the device path is tests/test_gpu_plugin_integration.py)."""
     import scenarios as S
-    if os.path.exists("/dev/nvidia0"):
-        pytest.skip("a CUDA device is present: covered by tests/test_gpu_plugin_integration.py")
+    monkeypatch.setenv("CUDA_VISIBLE_DEVICES", "")
     ops, opts = S.ALL["cfg2_mini"](per_run=300)
     want = H.run_reference(ops, **opts)
     got = H.run_reference(ops, binary=H.REF_B200_BIN, executor="b200", **opts)

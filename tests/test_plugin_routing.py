@@ -1,6 +1,7 @@
 """Which jobs the B200 executor plugin takes and which it leaves to the reference's CPU path (ShouldRunLocal,
 db/compaction/compaction_executor.h:162): decided from the job's options by WhyLocal() in toplingdb_b200/plugin/b200_compaction_executor.cc
-and reported, one line per job, when B200C_PLUGIN_TRACE is set.  The decision does not need a device, so it is checked here on the CPU:
+and reported, one line per job, when B200C_PLUGIN_TRACE is set.  The decision does not need a device, so it is checked here on the CPU,
+with any CUDA device hidden from the reference (a device would also run the jobs, and reject the data of some of them):
 every scenario of the GPU integration tests must be device-eligible (otherwise those tests would silently exercise the CPU path), and
 option shapes outside the device rule set must be recognised -- with the reference then producing its normal result."""
 import os
@@ -22,7 +23,7 @@ def _trace(fn, **extra):
         with open(os.path.join(d, "ops.bin"), "wb") as f:
             f.write(ops.bytes())
         args = [H.REF_B200_BIN, os.path.join(d, "ops.bin"), os.path.join(d, "w"), "executor=b200"] + [f"{k}={v}" for k, v in opts.items()]
-        r = subprocess.run(args, capture_output=True, text=True, env=dict(os.environ, B200C_PLUGIN_TRACE="1"))
+        r = subprocess.run(args, capture_output=True, text=True, env=dict(os.environ, B200C_PLUGIN_TRACE="1", CUDA_VISIBLE_DEVICES=""))
         assert r.returncode == 0, r.stderr[-2000:]
     lines = [ln for ln in r.stderr.splitlines() if ln.startswith("B200Compact: job ")]
     assert lines, "the executor factory was never asked"
